@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the vietTTS hot path on B200 (contract: see the task statement / DESIGN.md §Measurement).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[2], the one the metric is quoted on): per GPU a batch of 32
@@ -48,6 +48,26 @@ def peaks():
         return dict(hbm_gbs=d.get("hbm_gbs", 6650.0), bf16_tflops=d.get("bf16_tflops", 1590.0),
                     bf16_tflops_sustained=d.get("bf16_tflops_sustained", 1400.0), source="measured (MEASURED_PEAKS.json)")
     return dict(hbm_gbs=6650.0, bf16_tflops=1590.0, bf16_tflops_sustained=1400.0, source="fallback (B200_PROFILING.md)")
+
+
+DUMP_BUDGET_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays, budget=DUMP_BUDGET_BYTES):
+    """Writes each array as <out_dir>/<name>.npy in float32.  If together they exceed `budget` bytes, every array is
+    replaced by a flat sample of its elements (sorted indices drawn with a fixed seed from the array's size) of a size
+    proportional to its share, so that two builds run with the same arguments store the same positions."""
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float32) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    room = budget - 1024 * len(arrays)          # leaves room for the .npy headers
+    for name, a in arrays.items():
+        if total > room:
+            k = max(1, room * a.size // total)
+            idx = np.sort(np.random.default_rng(a.size).choice(a.size, size=k, replace=False))
+            a = a.reshape(-1)[idx]
+        np.save(out_dir / f"{name}.npy", a)
 
 
 def make_batch(batch: int, phonemes: int, seconds: float, seed0: int):
@@ -428,6 +448,8 @@ def run_ours(args):
         sampler.start()
     l0 = eng.launch_count()
     ms_step, ac_ms, hg_ms = time_jobs([job], args.steps, W, barrier)
+    # the last timed step's results, taken before the lines below run other work through the same buffers
+    dumped = dict(mel=job.mel_t.cpu().numpy(), wav=job.wav_t.cpu().numpy()) if args.dump_outputs and rank == 0 else None
     launches = (eng.launch_count() - l0) * args.steps // (args.steps + W)
     clocks = sampler.stop() if rank == 0 else None
     ms_step = allmax(ms_step)
@@ -642,6 +664,8 @@ def run_ours(args):
         )
         if world == 1 and not args.no_cpu:
             out["cpu_baseline"] = cpu_baseline(synthetic.hifigan_params(1234), synthetic.acoustic_ckpt(1234), args.phonemes, args.seconds)
+        if dumped is not None:
+            dump_outputs(args.dump_outputs, dumped)
         print(json.dumps(out))
     eng.close()
     if world > 1:
@@ -670,7 +694,14 @@ def main():
     ap.add_argument("--tc-variant", type=int, default=None, help="tile-shape variant of tc_conv (tuning aid; default: library default)")
     ap.add_argument("--precision", default="bf16x3", choices=["bf16x3", "fp32"],
                     help="conv arithmetic: bf16x3 = tcgen05 split-bf16 with fp32 accumulate (default), fp32 = FMA pipe")
+    ap.add_argument("--dump-outputs", type=Path, default=None, metavar="DIR",
+                    help="after the timed steps write what the last one computed for rank 0's batch, mel [B,N,80] and wav [B,256N], "
+                         "as DIR/mel.npy and DIR/wav.npy (float32, at most 64 MB in all: a fixed, seeded sample beyond that)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs records the CUDA path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

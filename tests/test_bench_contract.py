@@ -1,10 +1,13 @@
 """The bench.py JSON contract, checked on the committed record of the last B200 run (profiles/r2_bench_1gpu.json, or the
-round-1 record while that does not exist) and on the argument parser.  (The bench itself needs a GPU; the CPU reference
-arm is exercised by the driver.)"""
+round-1 record while that does not exist) and on the argument parser; the output dump of --dump-outputs on the host
+(writer, size budget) and, on the GPU, through a short bench run."""
 import json
 import subprocess
 import sys
 from pathlib import Path
+
+import numpy as np
+import pytest
 
 REPO = Path(__file__).resolve().parents[1]
 
@@ -49,5 +52,41 @@ def test_recorded_line_has_every_contract_key():
 def test_bench_cli_flags():
     out = subprocess.run([sys.executable, str(REPO / "bench.py"), "--help"], capture_output=True, text=True, timeout=120)
     assert out.returncode == 0
-    for flag in ("--gpus", "--steps", "--warmup", "--impl"):
+    for flag in ("--gpus", "--steps", "--warmup", "--impl", "--dump-outputs"):
         assert flag in out.stdout
+    bad = subprocess.run([sys.executable, str(REPO / "bench.py"), "--steps", "0"], capture_output=True, text=True, timeout=120)
+    assert bad.returncode != 0 and "--steps" in bad.stderr
+
+
+def test_dump_outputs_budget_and_sample(tmp_path):
+    import bench
+    rng = np.random.default_rng(0)
+    a, b = rng.standard_normal((3, 50, 8)), rng.standard_normal((3, 4000))
+    bench.dump_outputs(tmp_path / "whole", dict(mel=a, wav=b))
+    for name, x in (("mel", a), ("wav", b)):
+        got = np.load(tmp_path / "whole" / f"{name}.npy")
+        assert got.dtype == np.float32 and got.shape == x.shape and np.array_equal(got, x.astype(np.float32))
+    budget = 16 << 10                                   # smaller than the 52.8 kB the two arrays take
+    for run in ("s1", "s2"):
+        bench.dump_outputs(tmp_path / run, dict(mel=a, wav=b), budget=budget)
+    files = sorted((tmp_path / "s1").glob("*.npy"))
+    assert [f.name for f in files] == ["mel.npy", "wav.npy"] and sum(f.stat().st_size for f in files) <= budget
+    for f in files:
+        got, again = np.load(f), np.load(tmp_path / "s2" / f.name)
+        src = (a if f.stem == "mel" else b).astype(np.float32).reshape(-1)
+        assert got.dtype == np.float32 and got.ndim == 1 and 0 < got.size < src.size
+        assert np.array_equal(got, again) and np.isin(got, src).all()       # the same seeded positions every run
+
+
+@pytest.mark.gpu
+def test_bench_dumps_the_last_timed_step(tmp_path):
+    cmd = [sys.executable, str(REPO / "bench.py"), "--steps", "2", "--warmup", "1", "--batch", "2", "--no-cpu", "--no-callers",
+           "--no-sweep", "--no-configs", "--dump-outputs", str(tmp_path)]
+    out = subprocess.run(cmd, capture_output=True, text=True, timeout=900)
+    assert out.returncode == 0, out.stderr[-3000:]
+    d = json.loads(out.stdout.strip().splitlines()[-1])
+    assert d["steps"] == 2
+    n = d["config"]["mel_frames"]
+    mel, wav = np.load(tmp_path / "mel.npy"), np.load(tmp_path / "wav.npy")
+    assert mel.dtype == wav.dtype == np.float32 and mel.shape == (2, n, 80) and wav.shape == (2, 256 * n)
+    assert np.isfinite(mel).all() and np.isfinite(wav).all() and np.abs(wav).max() > 0

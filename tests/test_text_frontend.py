@@ -101,19 +101,3 @@ def test_pinned_buffers_are_released_with_the_array(monkeypatch):
     del view
     gc.collect()
     assert len(Engine._pinned_keepalive) == n0
-
-
-def test_golden_fixture_is_reproducible_where_the_reference_is_mounted(golden_dir, tmp_path):
-    """In the build container (/root/reference mounted) the committed fixture must be what the generator script
-    produces today from the reference's own functions; elsewhere (GPU box) this is skipped."""
-    import importlib.util
-    import pathlib
-    if not pathlib.Path("/root/reference/vietTTS/synthesizer.py").exists():
-        pytest.skip("reference tree not mounted")
-    spec = importlib.util.spec_from_file_location("make_text_golden", golden_dir / "make_text_golden.py")
-    gen = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(gen)
-    gen.OUT = tmp_path
-    gen.main()
-    assert json.loads((tmp_path / "text_frontend.json").read_text()) == json.loads((golden_dir / "text_frontend.json").read_text())
-    assert (tmp_path / "lexicon_small.txt").read_text() == (golden_dir / "lexicon_small.txt").read_text()
