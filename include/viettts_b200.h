@@ -136,12 +136,47 @@ int vtts_melspec(vtts_ctx* ctx, const float* wav_dev, int B, int S, float* mel_d
  * name: "enc" [B,L,512] (of the last acoustic OR duration call), "cond" [B,N,512], "mel_pre" [B,N,80] (before the postnet). */
 int vtts_debug_read(vtts_ctx* ctx, const char* name, float* host_out, int64_t n_floats);
 
-/* test hook: one hk.Conv1D (SAME padding, dilation, optional leaky_relu on the input and residual
- * add) on device buffers through either arithmetic path.  x [B,T,Cin], w Haiku layout [k,Cin,Cout],
- * out/resid [B,T,Cout]; len int32 [B] or NULL; pre_slope 1.0 = no input activation.  Synchronous. */
-int vtts_debug_conv1d(vtts_ctx* ctx, int precision, const float* x_dev, const float* w_dev, const float* bias_dev,
-                      const float* resid_dev, const int32_t* len_dev, int B, int T, int Cin, int Cout, int k, int dil,
-                      float pre_slope, float* out_dev);
+/* test hook: one conv launch of the models, run the way the models run it.  `geom` is the geometry every problem
+ * shares, `probs` 1..8 problems; all pointers are device memory.
+ *   input   x0 (and x1, x2 for pre_mode 2) [B][T_rows][Cin]; pre_mode 0 none, 1 leaky_relu(pre_slope),
+ *           2 leaky_relu(pre_slope) of (x0+x1+x2)/3
+ *   weights w Haiku layout [k][Cin][Cout], bias [Cout]; bn_mean / bn_inv / bn_off [Cout] all three or none:
+ *           y = (y - mean) * inv + off after the bias
+ *   output  post_act 0 none, 1 tanh, 2 relu after the BatchNorm, then + resid; out / resid [B][rows_out][Cout]
+ *   rows    output index tau reads input rows tau + j*dil + in_off (tap j, zero outside [0, valid_b)) and writes
+ *           output row tau*out_stride + out_off, for tau < valid_b = min(len[b]*len_mul, T_rows) (len NULL: T_rows).
+ *           Nothing else is written: output rows of tau >= valid_b keep their contents in both precisions.
+ * precision FP32: the strict fp32 conv (conv1d.cu).  BF16X3: every w packed by the loader's packer into N tiles of
+ * the width the models use, then the tensor-core dispatcher (tile width, partial last tile, epilogue form,
+ * launches of at most 8 tile problems).  Malformed descriptors (nprob outside 1..8, Cin % 16, Cout % 4, a partial
+ * BatchNorm triple, ...) return VTTS_ERR_BAD_ARG.  Synchronous. */
+typedef struct vtts_conv_geometry {
+  int32_t B, T_rows, rows_out, Cin, Cout;
+  const int32_t* len;
+  int32_t len_mul, pre_mode;
+  float pre_slope;
+  int32_t post_act;
+} vtts_conv_geometry;
+typedef struct vtts_conv_problem {
+  const float *x0, *x1, *x2;
+  const float* w;
+  const float* bias;
+  const float* resid;
+  const float *bn_mean, *bn_inv, *bn_off;
+  float* out;
+  int32_t k, dil, in_off, out_stride, out_off;
+} vtts_conv_problem;
+int vtts_debug_conv(vtts_ctx* ctx, int precision, const vtts_conv_geometry* geom, const vtts_conv_problem* probs, int nprob);
+
+/* test hook: one up-sampling stage of the generator, leaky_relu(0.1) -> hk.Conv1DTranspose(C/2, K, stride u, SAME)
+ * (vietTTS/hifigan/model.py:112-114), through the generator's own weight preparation and launch code.
+ * x0 [B][T][C]; x1, x2 NULL (stage 0: the input is x0) or both set (stages 1-3: the input is (x0+x1+x2)/3);
+ * w Haiku layout [K][C/2][C]; bias [C/2]; out [B][T*u][C/2]; len int32 [B] or NULL.  Output rows t = tau*u + r are
+ * written for tau < min(len[b]*len_mul, T), the others keep their contents.  (C, u, K) must be one of the generator's
+ * stages: (512, 8, 16), (256, 8, 16), (128, 2, 4), (64, 2, 4).  Synchronous. */
+int vtts_debug_conv_transpose(vtts_ctx* ctx, int precision, const float* x0_dev, const float* x1_dev, const float* x2_dev,
+                              const float* w_dev, const float* bias_dev, const int32_t* len_dev, int len_mul, int B, int T,
+                              int C, int u, int K, float* out_dev);
 
 /* test hook: one fused ResBlock pair  out = conv2(lrelu(conv1(lrelu(x)) + b1)) + b2 + x  (vietTTS/hifigan/model.py:44-51)
  * on the tensor-core path; x/out [B,T,C] with C in {32,64}, w1/w2 Haiku layout [k,C,C], conv1 dilation `dil`. Synchronous. */

@@ -189,7 +189,8 @@ def test_pinned_output_buffer_path(eng, hifigan_params):
 
 
 def test_batch_spanning_two_decoder_launches(eng, acoustic_ckpt):
-    """40 rows = two launches of the 32-row scan kernel: rows must not depend on their launch."""
+    """40 rows = one scan launch with two 32-row groups (up to 128 rows share a launch): rows must not depend on their
+    row group."""
     B = 40
     utts = [_utt(300 + b, 24, 0.6) for b in range(B)]
     L = 24

@@ -25,8 +25,9 @@ SIGNATURES = {
     "vtts_device_info": (C.c_int, [c_ctx, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int64)]),
     "vtts_set_precision": (C.c_int, [c_ctx, C.c_int]),
     "vtts_get_precision": (C.c_int, [c_ctx]),
-    "vtts_debug_conv1d": (C.c_int, [c_ctx, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
-                                    C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_void_p]),
+    "vtts_debug_conv": (C.c_int, [c_ctx, C.c_int, C.c_void_p, C.c_void_p, C.c_int]),
+    "vtts_debug_conv_transpose": (C.c_int, [c_ctx, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                            C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "vtts_debug_tc_stats": (C.c_int, [c_ctx, C.c_int, C.c_void_p]),
     "vtts_debug_substages": (C.c_int, [c_ctx, C.c_int, C.c_void_p]),
     "vtts_debug_pair": (C.c_int, [c_ctx, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
@@ -61,6 +62,19 @@ SIGNATURES = {
     "vtts_launch_count": (C.c_int64, [c_ctx]),
     "vtts_last_stage_ms": (C.c_int, [c_ctx, C.c_int, C.POINTER(C.c_float)]),
 }
+
+
+class ConvGeometry(C.Structure):
+    """vtts_conv_geometry"""
+    _fields_ = [("B", C.c_int32), ("T_rows", C.c_int32), ("rows_out", C.c_int32), ("Cin", C.c_int32), ("Cout", C.c_int32),
+                ("len", C.c_void_p), ("len_mul", C.c_int32), ("pre_mode", C.c_int32), ("pre_slope", C.c_float),
+                ("post_act", C.c_int32)]
+
+
+class ConvProblem(C.Structure):
+    """vtts_conv_problem"""
+    _fields_ = [(n, C.c_void_p) for n in ("x0", "x1", "x2", "w", "bias", "resid", "bn_mean", "bn_inv", "bn_off", "out")] + \
+               [(n, C.c_int32) for n in ("k", "dil", "in_off", "out_stride", "out_off")]
 
 
 class VttsError(RuntimeError):

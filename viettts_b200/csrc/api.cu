@@ -356,38 +356,81 @@ int vtts_debug_tc_stats(vtts_ctx* ctx, int enable, int64_t* host_out_256x16) {
   return VTTS_OK;
 }
 
-int vtts_debug_conv1d(vtts_ctx* ctx, int precision, const float* x_dev, const float* w_dev, const float* bias_dev,
-                      const float* resid_dev, const int32_t* len_dev, int B, int T, int Cin, int Cout, int k, int dil,
-                      float pre_slope, float* out_dev) {
+int vtts_debug_conv(vtts_ctx* ctx, int precision, const vtts_conv_geometry* geom, const vtts_conv_problem* probs, int nprob) {
   if (!ctx) return VTTS_ERR_BAD_ARG;
+  if (precision != VTTS_PRECISION_FP32 && precision != VTTS_PRECISION_BF16X3) return ctx->fail(VTTS_ERR_BAD_ARG, "debug_conv: precision %d", precision);
+  if (!geom || !probs || nprob < 1 || nprob > 8) return ctx->fail(VTTS_ERR_BAD_ARG, "debug_conv: nprob %d", nprob);
+  const vtts_conv_geometry& g = *geom;
+  if (g.Cin < 16 || g.Cin % 16 != 0 || g.Cout < 4 || g.Cout % 4 != 0) return ctx->fail(VTTS_ERR_BAD_ARG, "debug_conv: Cin %d / Cout %d", g.Cin, g.Cout);
+  if (g.B < 1 || g.T_rows < 1 || g.rows_out < 1 || g.len_mul < 1 || g.pre_mode < 0 || g.pre_mode > 2 || g.post_act < 0 || g.post_act > 2)
+    return ctx->fail(VTTS_ERR_BAD_ARG, "debug_conv: B %d T_rows %d rows_out %d len_mul %d pre_mode %d post_act %d", g.B, g.T_rows,
+                     g.rows_out, g.len_mul, g.pre_mode, g.post_act);
+  ConvLaunch L;
+  memset(&L, 0, sizeof(L));
+  L.nprob = nprob; L.Cin = g.Cin; L.Cout = g.Cout; L.B = g.B; L.T_rows = g.T_rows; L.rows_out = g.rows_out;
+  L.len = g.len; L.len_mul = g.len_mul; L.pre_mode = g.pre_mode; L.pre_slope = g.pre_slope; L.post_act = g.post_act;
+  for (int i = 0; i < nprob; ++i) {
+    const vtts_conv_problem& q = probs[i];
+    const int nbn = (q.bn_mean != nullptr) + (q.bn_inv != nullptr) + (q.bn_off != nullptr);
+    // x1 and x2 go together, and exactly with pre_mode 2 (as in vtts_debug_conv_transpose)
+    if (!q.x0 || !q.w || !q.bias || !q.out || (nbn != 0 && nbn != 3) || (q.x1 == nullptr) != (q.x2 == nullptr) ||
+        (q.x1 != nullptr) != (g.pre_mode == 2))
+      return ctx->fail(VTTS_ERR_BAD_ARG, "debug_conv: problem %d: missing pointer, partial BatchNorm, or x1/x2 not both set with pre_mode 2", i);
+    if (q.k < 1 || q.dil < 1 || q.out_stride < 1 || q.out_off < 0 || (int64_t)(g.T_rows - 1) * q.out_stride + q.out_off >= g.rows_out)
+      return ctx->fail(VTTS_ERR_BAD_ARG, "debug_conv: problem %d: k %d dil %d out_stride %d out_off %d", i, q.k, q.dil, q.out_stride, q.out_off);
+    L.p[i] = ConvProb{q.x0, q.x1, q.x2, q.w, q.bias, q.resid, q.bn_mean, q.bn_inv, q.bn_off, q.out, q.k, q.dil, q.in_off, q.out_stride, q.out_off};
+  }
   VTTS_CUDA(cudaSetDevice(ctx->device));
   if (precision == VTTS_PRECISION_FP32) {
-    ConvLaunch L;
-    memset(&L, 0, sizeof(L));
-    L.nprob = 1; L.Cin = Cin; L.Cout = Cout; L.B = B; L.T_rows = T; L.rows_out = T; L.len = len_dev; L.len_mul = 1;
-    L.pre_mode = pre_slope == 1.0f ? 0 : 1; L.pre_slope = pre_slope; L.post_act = 0;
-    L.p[0] = ConvProb{x_dev, nullptr, nullptr, w_dev, bias_dev, resid_dev, nullptr, nullptr, nullptr, out_dev, k, dil, -((k - 1) * dil) / 2, 1, 0};
     int rc = vtts_launch_conv(ctx, L, nullptr);
     if (rc) return rc;
-  } else {
-    void* wpk = nullptr;
-    VTTS_CUDA(cudaMalloc(&wpk, vtts_tc_packed_elems(k, Cin, Cout) * 2));
-    int rc = vtts_tc_pack_weights(ctx, w_dev, wpk, k, Cin, Cout, 0, Cout);
-    if (rc) { cudaFree(wpk); return rc; }
-    TcLaunch TL;
-    memset(&TL, 0, sizeof(TL));
-    TL.nprob = 1; TL.Cin = Cin; TL.N = Cout; TL.in_ld = Cin; TL.out_ld = Cout; TL.B = B; TL.T_rows = T; TL.rows_out = T;
-    TL.len = len_dev; TL.len_mul = 1; TL.pre_mode = pre_slope == 1.0f ? 0 : 1; TL.pre_slope = pre_slope;
-    TL.p[0] = TcProb{x_dev, nullptr, nullptr, wpk, bias_dev, resid_dev, nullptr, nullptr, nullptr, out_dev, k, dil, -((k - 1) * dil) / 2, 1, 0};
-    rc = vtts_launch_tc_conv(ctx, TL, nullptr);
-    cudaError_t e = cudaDeviceSynchronize();
-    cudaFree(wpk);
-    if (rc) return rc;
-    if (e != cudaSuccess) {
-      return ctx->fail(VTTS_ERR_CUDA, "debug_conv1d (tensor path): %s", cudaGetErrorString(e));
-    }
+    VTTS_CUDA(cudaDeviceSynchronize());
+    return VTTS_OK;
   }
-  VTTS_CUDA(cudaDeviceSynchronize());
+  size_t bytes = 0;
+  for (int i = 0; i < nprob; ++i) bytes += vtts_tc_conv_packed_bytes(L.p[i].k, g.Cin, g.Cout);
+  void* pk = nullptr;
+  VTTS_CUDA(cudaMalloc(&pk, bytes));
+  std::vector<void*> wpk;   // wpk[prob * ntile + tile], the order vtts_conv_dispatch reads
+  char* cur = (char*)pk;
+  int rc = VTTS_OK;
+  for (int i = 0; i < nprob && !rc; ++i) rc = vtts_tc_pack_conv(ctx, L.p[i].w, L.p[i].k, g.Cin, g.Cout, cur, wpk);
+  const int saved = ctx->precision;
+  ctx->precision = VTTS_PRECISION_BF16X3;     // the dispatcher takes the tensor-core path in this mode only; restored below
+  if (!rc) rc = vtts_conv_dispatch(ctx, L, wpk.data(), nullptr);
+  ctx->precision = saved;
+  cudaError_t e = cudaDeviceSynchronize();
+  cudaFree(pk);
+  if (rc) return rc;
+  if (e != cudaSuccess) return ctx->fail(VTTS_ERR_CUDA, "debug_conv (tensor path): %s", cudaGetErrorString(e));
+  return VTTS_OK;
+}
+
+int vtts_debug_conv_transpose(vtts_ctx* ctx, int precision, const float* x0_dev, const float* x1_dev, const float* x2_dev,
+                              const float* w_dev, const float* bias_dev, const int32_t* len_dev, int len_mul, int B, int T,
+                              int C, int u, int K, float* out_dev) {
+  if (!ctx) return VTTS_ERR_BAD_ARG;
+  if (precision != VTTS_PRECISION_FP32 && precision != VTTS_PRECISION_BF16X3) return ctx->fail(VTTS_ERR_BAD_ARG, "debug_conv_transpose: precision %d", precision);
+  bool stage = false;
+  for (int i = 0, c = vc::HG_C0; i < vc::HG_NSTAGE; ++i, c /= 2) stage |= C == c && u == vc::hg_rate(i) && K == vc::hg_upk(i);
+  if (!stage) return ctx->fail(VTTS_ERR_BAD_ARG, "debug_conv_transpose: (C %d, u %d, K %d) is not a generator stage", C, u, K);
+  if (!x0_dev || !w_dev || !bias_dev || !out_dev || (x1_dev == nullptr) != (x2_dev == nullptr))
+    return ctx->fail(VTTS_ERR_BAD_ARG, "debug_conv_transpose: missing pointer (x1 and x2 go together)");
+  if (B < 1 || T < 1 || len_mul < 1 || (int64_t)T * u > INT32_MAX / 64) return ctx->fail(VTTS_ERR_BAD_ARG, "debug_conv_transpose: B %d T %d len_mul %d", B, T, len_mul);
+  VTTS_CUDA(cudaSetDevice(ctx->device));
+  const size_t upsw_bytes = ((size_t)u * 2 * C * (C / 2) * sizeof(float) + 255) & ~size_t(255);
+  const size_t ph_bytes = (vtts_tc_packed_elems(2, C, C / 2) * 2 + 255) & ~size_t(255);
+  char* buf = nullptr;
+  VTTS_CUDA(cudaMalloc(&buf, upsw_bytes + u * ph_bytes));
+  void* wpk[8];
+  for (int r = 0; r < u; ++r) wpk[r] = buf + upsw_bytes + r * ph_bytes;
+  int rc = vtts_hg_ups_prepare(ctx, w_dev, C, u, K, (float*)buf, wpk);
+  if (!rc) rc = vtts_hg_ups_run(ctx, precision == VTTS_PRECISION_BF16X3, x0_dev, x1_dev, x2_dev, (const float*)buf, wpk, bias_dev,
+                                len_dev, len_mul, B, T, C, u, K, out_dev, nullptr);
+  cudaError_t e = cudaDeviceSynchronize();
+  cudaFree(buf);
+  if (rc) return rc;
+  if (e != cudaSuccess) return ctx->fail(VTTS_ERR_CUDA, "debug_conv_transpose: %s", cudaGetErrorString(e));
   return VTTS_OK;
 }
 

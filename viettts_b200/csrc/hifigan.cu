@@ -108,6 +108,68 @@ size_t vtts_hifigan_ws_bytes(int B, int T) {
   return ar.off + 256;
 }
 
+int vtts_hg_ups_prepare(vtts_ctx* ctx, const float* w, int C, int u, int K, float* upsw, void* const* wpk) {
+  const int Co = C / 2, a = (K + u - 2 + 1) / 2;
+  repack_ups_kernel<<<256, 256>>>(w, upsw, u, K, C, Co, a);
+  VTTS_CUDA(cudaGetLastError());
+  // (same stream as the repack: the phase weights are packed from upsw after it is complete)
+  for (int r = 0; r < u; ++r) {
+    int rc = vtts_tc_pack_weights(ctx, upsw + (size_t)r * 2 * C * Co, wpk[r], 2, C, Co, 0, Co);
+    if (rc) return rc;
+  }
+  return VTTS_OK;
+}
+
+int vtts_hg_ups_run(vtts_ctx* ctx, bool tc, const float* x0, const float* x1, const float* x2, const float* upsw,
+                    void* const* wpk, const float* bias, const int32_t* len, int len_mul, int B, int T, int C, int u, int K,
+                    float* out, cudaStream_t st) {
+  const int Co = C / 2;
+  const int a = (K + u - 2 + 1) / 2;
+  ConvLaunch L;
+  memset(&L, 0, sizeof(L));
+  L.B = B; L.len = len; L.len_mul = len_mul;
+  L.nprob = u; L.Cin = C; L.Cout = Co;
+  L.T_rows = T; L.rows_out = T * u;
+  L.pre_mode = x1 ? 2 : 1; L.pre_slope = 0.1f; L.post_act = 0;
+  for (int r = 0; r < u; ++r) {
+    int j0 = ((a - r) % u + u) % u;
+    int e = (r + j0 - a) / u;  // exact division, <= 0
+    ConvProb p;
+    memset(&p, 0, sizeof(p));
+    p.x0 = x0; p.x1 = x1; p.x2 = x2;
+    p.w = upsw + (size_t)r * 2 * C * Co;
+    p.bias = bias;
+    p.out = out;
+    p.k = 2; p.dil = 1; p.in_off = e; p.out_stride = u; p.out_off = r;
+    L.p[r] = p;
+  }
+  if (!tc) return vtts_launch_conv(ctx, L, st);
+  // ConvTranspose phases share their input: for N <= 128 one converted activation tile feeds NPH phases
+  // (multi-phase tiles of tc_conv.cu); N = 256 keeps one problem per phase.
+  const int nph = Co == 256 ? 1 : (Co == 128 ? 4 : 2);
+  TcLaunch TL;
+  memset(&TL, 0, sizeof(TL));
+  TL.nprob = u / nph; TL.nphase = nph; TL.Cin = C; TL.N = Co; TL.in_ld = C; TL.out_ld = Co;
+  TL.B = B; TL.T_rows = T; TL.rows_out = T * u; TL.len = len; TL.len_mul = len_mul;
+  TL.pre_mode = L.pre_mode; TL.pre_slope = 0.1f;
+  for (int g = 0; g < u / nph; ++g) {
+    const ConvProb& c0 = L.p[g * nph];
+    TcProb q;
+    memset(&q, 0, sizeof(q));
+    q.x0 = c0.x0; q.x1 = c0.x1; q.x2 = c0.x2; q.bias = c0.bias; q.out = c0.out;
+    q.k = 2; q.dil = 1; q.out_stride = u;
+    q.wpk = wpk[g * nph]; q.in_off = c0.in_off; q.out_off = g * nph;
+    for (int ph = 0; ph < nph; ++ph) {
+      const int r = g * nph + ph;
+      q.wpk_ph[ph] = wpk[r];
+      q.in_off_ph[ph] = L.p[r].in_off;
+      q.out_off_ph[ph] = r;
+    }
+    TL.p[g] = q;
+  }
+  return vtts_launch_tc_conv(ctx, TL, st);
+}
+
 int vtts_hifigan_prepare(vtts_ctx* ctx) {
   // repacked transposed-conv weights
   size_t total = 0;
@@ -120,17 +182,8 @@ int vtts_hifigan_prepare(vtts_ctx* ctx) {
   }
   if (ctx->hg_upsw) cudaFree(ctx->hg_upsw);
   VTTS_CUDA(cudaMalloc(&ctx->hg_upsw, total * sizeof(float)));
-  C = vc::HG_C0;
-  for (int i = 0; i < 4; ++i) {
-    int u = vc::hg_rate(i), K = vc::hg_upk(i);
-    int a = (K + u - 2 + 1) / 2;
-    repack_ups_kernel<<<256, 256>>>(ctx->hg_t[hgi::UPS_W(i)], ctx->hg_upsw + offs[i], u, K, C, C / 2, a);
-    VTTS_CUDA(cudaGetLastError());
-    C /= 2;
-  }
   // ---- tensor-core path: bf16 hi/lo split + canonical K-major packing of every dense conv ----
   {
-    VTTS_CUDA(cudaDeviceSynchronize());  // hg_upsw must be complete: the phase weights are packed from it
     size_t elems = 0;
     std::vector<size_t> eoff(72), uoff(32), poff(2);
     for (int n = 0; n < 12; ++n) {
@@ -190,13 +243,11 @@ int vtts_hifigan_prepare(vtts_ctx* ctx) {
     }
     Cc = vc::HG_C0;
     for (int i = 0; i < 4; ++i) {
-      const int Co = Cc / 2;
-      for (int r = 0; r < vc::hg_rate(i); ++r) {
-        ctx->hg_wpk_ups[i * 8 + r] = (char*)ctx->hg_wpk + uoff[i * 8 + r] * 2;
-        int rc = vtts_tc_pack_weights(ctx, ctx->hg_upsw + offs[i] + (size_t)r * 2 * Cc * Co, ctx->hg_wpk_ups[i * 8 + r], 2, Cc, Co, 0, Co);
-        if (rc) return rc;
-      }
-      Cc = Co;
+      for (int r = 0; r < vc::hg_rate(i); ++r) ctx->hg_wpk_ups[i * 8 + r] = (char*)ctx->hg_wpk + uoff[i * 8 + r] * 2;
+      int rc = vtts_hg_ups_prepare(ctx, ctx->hg_t[hgi::UPS_W(i)], Cc, vc::hg_rate(i), vc::hg_upk(i), ctx->hg_upsw + offs[i],
+                                   &ctx->hg_wpk_ups[i * 8]);
+      if (rc) return rc;
+      Cc /= 2;
     }
     for (int t = 0; t < 2; ++t) {
       ctx->hg_wpk_pre[t] = (char*)ctx->hg_wpk + poff[t] * 2;
@@ -250,57 +301,17 @@ int vtts_hifigan_run(vtts_ctx* ctx, const float* mel, const int32_t* n_frames, i
   int C = vc::HG_C0;      // input channels of the stage
   int rows_in = T;        // rows per batch item entering the stage
   int scale_in = 1;       // rows_in = T*scale_in
-  size_t ups_off = 0;
+  size_t ups_off = 0;     // offset of the stage's phase weights in ctx->hg_upsw
   for (int i = 0; i < 4; ++i) {
     const int u = vc::hg_rate(i), K = vc::hg_upk(i), Co = C / 2;
-    const int a = (K + u - 2 + 1) / 2;
     const int par = i & 1;
     // ---- lrelu(0.1) [of the 3-way mean for i>0] -> ConvTranspose as u two-tap phases ----
-    memset(&L, 0, sizeof(L));
-    L.B = B; L.len = n_frames; L.len_mul = scale_in;
-    L.nprob = u; L.Cin = C; L.Cout = Co;
-    L.T_rows = rows_in; L.rows_out = rows_in * u;
-    L.pre_mode = (i == 0) ? 1 : 2; L.pre_slope = 0.1f; L.post_act = 0;
-    for (int r = 0; r < u; ++r) {
-      int j0 = ((a - r) % u + u) % u;
-      int e = (r + j0 - a) / u;  // exact division, <= 0
-      ConvProb p;
-      memset(&p, 0, sizeof(p));
-      if (i == 0) { p.x0 = hb.P0; } else { p.x0 = hb.A[par ^ 1][0]; p.x1 = hb.A[par ^ 1][1]; p.x2 = hb.A[par ^ 1][2]; }
-      p.w = ctx->hg_upsw + ups_off + (size_t)r * 2 * C * Co;
-      p.bias = W[hgi::UPS_B(i)];
-      p.out = hb.X;
-      p.k = 2; p.dil = 1; p.in_off = e; p.out_stride = u; p.out_off = r;
-      L.p[r] = p;
-    }
-    if (tc) {
-      // ConvTranspose phases share their input: for N <= 128 one converted activation tile feeds NPH phases
-      // (multi-phase tiles of tc_conv.cu); N = 256 keeps one problem per phase.
-      const int nph = Co == 256 ? 1 : (Co == 128 ? 4 : 2);
-      TcLaunch TL;
-      memset(&TL, 0, sizeof(TL));
-      TL.nprob = u / nph; TL.nphase = nph; TL.Cin = C; TL.N = Co; TL.in_ld = C; TL.out_ld = Co;
-      TL.B = B; TL.T_rows = rows_in; TL.rows_out = rows_in * u; TL.len = n_frames; TL.len_mul = scale_in;
-      TL.pre_mode = L.pre_mode; TL.pre_slope = 0.1f;
-      for (int g = 0; g < u / nph; ++g) {
-        const ConvProb& c0 = L.p[g * nph];
-        TcProb q;
-        memset(&q, 0, sizeof(q));
-        q.x0 = c0.x0; q.x1 = c0.x1; q.x2 = c0.x2; q.bias = c0.bias; q.out = c0.out;
-        q.k = 2; q.dil = 1; q.out_stride = u;
-        q.wpk = ctx->hg_wpk_ups[i * 8 + g * nph]; q.in_off = c0.in_off; q.out_off = g * nph;
-        for (int ph = 0; ph < nph; ++ph) {
-          const int r = g * nph + ph;
-          q.wpk_ph[ph] = ctx->hg_wpk_ups[i * 8 + r];
-          q.in_off_ph[ph] = L.p[r].in_off;
-          q.out_off_ph[ph] = r;
-        }
-        TL.p[g] = q;
-      }
-      rc = vtts_launch_tc_conv(ctx, TL, st);
-    } else {
-      rc = vtts_launch_conv(ctx, L, st);
-    }
+    if (i == 0)
+      rc = vtts_hg_ups_run(ctx, tc, hb.P0, nullptr, nullptr, ctx->hg_upsw + ups_off, &ctx->hg_wpk_ups[i * 8], W[hgi::UPS_B(i)],
+                           n_frames, scale_in, B, rows_in, C, u, K, hb.X, st);
+    else
+      rc = vtts_hg_ups_run(ctx, tc, hb.A[par ^ 1][0], hb.A[par ^ 1][1], hb.A[par ^ 1][2], ctx->hg_upsw + ups_off,
+                           &ctx->hg_wpk_ups[i * 8], W[hgi::UPS_B(i)], n_frames, scale_in, B, rows_in, C, u, K, hb.X, st);
     if (rc) return rc;
     ups_off += (size_t)u * 2 * C * Co;
 

@@ -571,6 +571,8 @@ int launch_cfg(vtts_ctx* ctx, TcLaunch& L, cudaStream_t st) {
 
 // tile shapes: single-phase: N=256 -> MT 1, N=128 -> MT 2 (two accumulator sets), N<=64 -> MT 4
 //              multi-phase (ConvTranspose): N=128 x 4 phases x MT 1, N=64 x 2 x MT 2, N=32 x 2 x MT 4
+// (tests/test_gpu_conv_configs.py _tile_rows restates the default-variant shapes to place its rows on tile edges: keep
+//  the two in step)
 template <int N, int EPI>
 int launch_ne(vtts_ctx* ctx, TcLaunch& L, cudaStream_t st) {
   const int nph = L.nphase > 1 ? L.nphase : 1;

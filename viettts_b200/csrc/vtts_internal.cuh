@@ -278,6 +278,15 @@ size_t vtts_tc_conv_packed_bytes(int k, int Cin, int Cout);
 int vtts_hifigan_prepare(vtts_ctx* ctx);   // derived weights after load
 int vtts_hifigan_run(vtts_ctx* ctx, const float* mel, const int32_t* n_frames, int B, int T, float* wav, cudaStream_t st);
 size_t vtts_hifigan_ws_bytes(int B, int T);
+// one up-sampling stage (C -> C/2 channels, rate u, kernel K) of the generator; vtts_debug_conv_transpose runs the same two.
+// prepare: Haiku w[K][C/2][C] -> per output phase r the two-tap conv weight upsw[r] = [2][C][C/2] (fp32 path, u*2*C*C/2
+//          floats) and its packed tensor-core copy wpk[r] (vtts_tc_packed_elems(2, C, C/2) bf16 each)
+// run:     lrelu(0.1)(x0), or lrelu(0.1)((x0+x1+x2)/3) when x1 != null, -> ConvTranspose as u phases: x [B][T][C] ->
+//          out [B][T*u][C/2], rows tau*u + r written for tau < min(len[b]*len_mul, T); tc selects the tensor-core path
+int vtts_hg_ups_prepare(vtts_ctx* ctx, const float* w, int C, int u, int K, float* upsw, void* const* wpk);
+int vtts_hg_ups_run(vtts_ctx* ctx, bool tc, const float* x0, const float* x1, const float* x2, const float* upsw,
+                    void* const* wpk, const float* bias, const int32_t* len, int len_mul, int B, int T, int C, int u, int K,
+                    float* out, cudaStream_t st);
 // nat.cu
 int vtts_acoustic_prepare(vtts_ctx* ctx);
 int vtts_acoustic_run(vtts_ctx* ctx, const int32_t* tokens, const int32_t* lengths, const float* dur,

@@ -89,15 +89,40 @@ class Engine:
         self._ck(self.lib.vtts_set_precision(self.h, int(m)))
 
     def debug_conv1d(self, precision, x_t, w_t, bias_t, k, dil, pre_slope=1.0, resid_t=None, len_t=None):
-        """Test hook: one conv layer on torch CUDA tensors through either arithmetic path."""
+        """Test hook: one conv layer (SAME padding, leaky_relu(pre_slope) on the input unless pre_slope == 1, optional
+        residual) on torch CUDA tensors through either arithmetic path; x [B,T,Cin], w [k,Cin,Cout] -> [B,T,Cout]."""
         import torch
         B, T, Cin = x_t.shape
-        Cout = w_t.shape[2]
-        out = torch.empty((B, T, Cout), dtype=torch.float32, device=x_t.device)
-        m = {"fp32": PRECISION_FP32, "bf16x3": PRECISION_BF16X3}.get(precision, precision)
-        self._ck(self.lib.vtts_debug_conv1d(self.h, int(m), _ptr(x_t), _ptr(w_t), _ptr(bias_t), _ptr(resid_t), _ptr(len_t),
-                                            B, T, Cin, Cout, int(k), int(dil), float(pre_slope), _ptr(out)))
+        out = torch.empty((B, T, w_t.shape[2]), dtype=torch.float32, device=x_t.device)
+        self.debug_conv(precision, [dict(x0=x_t, w=w_t, bias=bias_t, resid=resid_t, out=out, k=k, dil=dil, in_off=-((k - 1) * dil // 2))],
+                        B=B, T_rows=T, rows_out=T, Cin=Cin, Cout=w_t.shape[2], len_t=len_t,
+                        pre_mode=0 if pre_slope == 1.0 else 1, pre_slope=pre_slope)
         return out
+
+    _CONV_PTRS = ("x0", "x1", "x2", "w", "bias", "resid", "bn_mean", "bn_inv", "bn_off", "out")
+
+    def debug_conv(self, precision, problems, *, B, T_rows, rows_out, Cin, Cout, len_t=None, len_mul=1, pre_mode=0, pre_slope=1.0,
+                   post_act=0):
+        """Test hook vtts_debug_conv: one conv launch of up to 8 problems through the models' own dispatch.  `problems`
+        is a list of dicts with torch CUDA tensors under x0, x1, x2, w, bias, resid, bn_mean, bn_inv, bn_off, out (absent =
+        NULL) and the ints k, dil, in_off, out_stride (default 1), out_off (default 0).  Writes the `out` tensors."""
+        m = {"fp32": PRECISION_FP32, "bf16x3": PRECISION_BF16X3}.get(precision, precision)
+        geom = _lib.ConvGeometry(B, T_rows, rows_out, Cin, Cout, _ptr(len_t), len_mul, pre_mode, pre_slope, post_act)
+        probs = (_lib.ConvProblem * max(1, len(problems)))()
+        for p, d in zip(probs, problems):
+            for name in self._CONV_PTRS:
+                setattr(p, name, _ptr(d.get(name)))
+            p.k, p.dil, p.in_off = int(d["k"]), int(d["dil"]), int(d["in_off"])
+            p.out_stride, p.out_off = int(d.get("out_stride", 1)), int(d.get("out_off", 0))
+        self._ck(self.lib.vtts_debug_conv(self.h, int(m), C.byref(geom), probs, len(problems)))
+
+    def debug_conv_transpose(self, precision, x0_t, w_t, bias_t, out_t, u, x1_t=None, x2_t=None, len_t=None, len_mul=1):
+        """Test hook vtts_debug_conv_transpose: one generator up-sampling stage, lrelu(0.1) of x0 (or of (x0+x1+x2)/3)
+        -> ConvTranspose(stride u); x [B,T,C], w Haiku [K,C/2,C] -> out_t [B,T*u,C/2] (rows past len*len_mul*u untouched)."""
+        m = {"fp32": PRECISION_FP32, "bf16x3": PRECISION_BF16X3}.get(precision, precision)
+        B, T, Cc = x0_t.shape
+        self._ck(self.lib.vtts_debug_conv_transpose(self.h, int(m), _ptr(x0_t), _ptr(x1_t), _ptr(x2_t), _ptr(w_t), _ptr(bias_t),
+                                                    _ptr(len_t), int(len_mul), B, T, Cc, int(u), int(w_t.shape[0]), _ptr(out_t)))
 
     def debug_pair(self, x_t, w1_t, b1_t, w2_t, b2_t, k, dil, slope=0.1, len_t=None):
         """Test hook: one fused ResBlock pair on torch CUDA tensors (tensor-core path)."""
